@@ -1,66 +1,34 @@
 """Header processing inside the library (csrc/xm_headers.h: xm_process_headers_fds / _mem) against the reference's
 get_sam_header / add_pg_tag / process_headers (xm.py:36-46, 120-174): same six header texts, same errors, and the byte
-offset of the first record.  The reference itself is used when /root/reference is present (this container); the
-package's Python text path -- pinned to the reference by the golden tests -- otherwise."""
-import io
+offset of the first record.  The text layer's answers are stored in tests/golden/headers.json
+(tests/golden/make_header_golden.py); the package's Python text path must still give them too."""
+import json
 import os
-import sys
 
 import pytest
 
+from tests._header_cases import CASES, ENABLED, H1, H2, NAMES, REC, key, text_layer
 from xenomapper_b200 import _lib
 from xenomapper_b200 import xenomapper as xm
 
-REC = "r1\t0\tchr1\t1\t42\t5M\t*\t0\t0\tACGTA\tFFFFF\tAS:i:10\n"
-H1 = "@HD\tVN:1.0\tSO:unsorted\n@SQ\tSN:chr1\tLN:1000\n@PG\tID:bowtie2\tPN:bowtie2\tVN:2.2.6\tCL:\"bowtie2-align-s --local\"\n"
-H2 = "@HD\tVN:1.0\n@SQ\tSN:1\tLN:500\n"
-NAMES = ("primary_specific", "secondary_specific", "primary_multi", "secondary_multi", "unassigned", "unresolved")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "headers.json")
 
 
-def reference_module():
-    if os.path.isdir("/root/reference/xenomapper"):
-        sys.path.insert(0, "/root/reference")
-        try:
-            from xenomapper import xenomapper as ref
-            return ref
-        finally:
-            sys.path.pop(0)
-    return xm          # the Python text path of the package (StringIO inputs never take the native route)
+def expected(name, enabled):
+    """the stored answer of the text layer; the package's Python text path (StringIO inputs never take the native
+    route) must give the same"""
+    with open(GOLDEN, encoding="utf-8") as f:
+        a = json.load(f)["answers"][key(name, enabled)]
+    want = a["error"], a["headers"], a["rest"]
+    assert text_layer(xm, *CASES[name], enabled) == want, "the Python text layer no longer gives the stored answer"
+    return want
 
 
-def expected(text1, text2, enabled):
-    """(exception class or None, six header strings, remaining text of both inputs) from the text-layer implementation"""
-    ref = reference_module()
-    f1, f2 = io.StringIO(text1, newline=None), io.StringIO(text2, newline=None)
-    outs = {n: (io.StringIO() if (enabled >> b) & 1 or b == 0 else None) for b, n in enumerate(NAMES)}
-    try:
-        ref.process_headers(f1, f2, **outs)
-    except Exception as e:                                       # noqa: BLE001 -- the class is what is compared
-        return type(e), None, None
-    return None, [outs[n].getvalue() if outs[n] else None for n in NAMES], (f1.read(), f2.read())
-
-
-CASES = {
-    "plain": (H1 + REC, H2 + REC),
-    "crlf": ((H1 + REC).replace("\n", "\r\n"), H2 + REC),
-    "lone_cr_in_header": (H1.replace("\n", "\r") + REC, H2 + REC),
-    "no_header": (REC, H2 + REC),
-    "empty": ("", H2 + REC),
-    "header_only": (H1, H2 + REC),
-    "blank_line_after_header": (H1 + "\n" + REC, H2 + REC),
-    "pg_without_id": (H1, "@HD\tVN:1.0\n@PG\tPN:bowtie2\n" + REC),
-    "pg_id_after_unicode_space": (H1 + REC, "@HD\tVN:1.0\n@PG\tPN:x ID:abc VN:1\n" + REC),
-    "pg_not_last": (H1 + "@CO\tsomething\n" + REC, H2 + REC),
-    "non_ascii_header": (H1 + REC, "@CO\tnaïve café\n" + REC),
-    "secondary_header_only": (H1 + REC, H2),
-}
-
-
-@pytest.mark.parametrize("enabled", [0x3F, 0x01, 0x15], ids=["all", "primary_specific_only", "primary_bins"])
+@pytest.mark.parametrize("enabled", list(ENABLED.values()), ids=list(ENABLED))
 @pytest.mark.parametrize("name", list(CASES))
 def test_native_headers_match_the_text_layer(tmp_path, name, enabled):
     t1, t2 = CASES[name]
-    err, texts, rest = expected(t1, t2, enabled)
+    err, texts, rest = expected(name, enabled)
     b1, b2 = t1.encode(), t2.encode()
     for route in ("mem", "fds"):
         if route == "mem":
@@ -73,14 +41,14 @@ def test_native_headers_match_the_text_layer(tmp_path, name, enabled):
             [os.close(f) for f in fds]
         first_error = None
         if rc == _lib.XM_ERR_INDEX:
-            first_error = IndexError
+            first_error = "IndexError"
         elif rc == _lib.XM_ERR_UNICODE:
-            first_error = UnicodeDecodeError
+            first_error = "UnicodeDecodeError"
         else:
             assert rc == 0
             for b in range(6):
                 if ((enabled >> b) & 1 or b == 0) and status[b] == _lib.XM_ERR_INDEX:
-                    first_error = IndexError
+                    first_error = "IndexError"
                     break
         assert first_error == err, (route, rc, status)
         if err is None:
