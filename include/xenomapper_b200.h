@@ -309,7 +309,7 @@ typedef struct xm_bam_stats {
     float render_ms;         /* device time of the three BAM text kernels */
     uint32_t n_launches;
     uint64_t bam_bytes, inflated_bytes, text_bytes, records;
-    double upload_s;         /* of inflate_s: pageable host memory -> device (the compressed bytes) */
+    double upload_s;         /* of inflate_s: pageable host memory -> device (the compressed bytes; XM_BAM_INFLATE=host: the inflated ones) */
     float inflate_ms;        /* device time of k_bgzf_inflate */
     uint32_t chain_repairs;  /* segments of the record chain whose guessed entry was not the true one */
 } xm_bam_stats;

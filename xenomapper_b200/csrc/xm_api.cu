@@ -203,8 +203,7 @@ struct xm_ctx {
     std::vector<Block> bins[6];
     std::vector<uint8_t> flat[6];       /* xm_get_output of a bin that spans several blocks */
     uint64_t block_bytes = 0;
-    /* BAM input: inflated streams (pinned), device copies, record tables, rendered SAM text */
-    HostBuf h_bam[2];
+    /* BAM input: inflated windows, record tables, rendered SAM text */
     DevBuf d_bam[2], d_bam_rec[2], d_bam_ref[2], d_bam_len[2], d_bam_sum[2], d_bam_text[2];
     DevBuf d_bam_comp[2], d_bam_tab[2], d_bam_seg[2];      /* compressed window, its block table, the chain's segments */
     /* BGZF output deflated on the device (xm_deflate.h): member slots, sizes + offsets + plan, packed members per output set and bin */
@@ -301,7 +300,6 @@ void xm_destroy(xm_ctx *c)
     for (auto &s : c->d_out) for (auto &b : s) if (b.p) cudaFree(b.p);
     for (auto &b : c->h_stage) if (b.p) cudaFreeHost(b.p);
     bam_shard_free(c);
-    for (auto &b : c->h_bam) if (b.p) cudaFreeHost(b.p);
     if (c->d_zslot.p) cudaFree(c->d_zslot.p);
     if (c->d_zmeta.p) cudaFree(c->d_zmeta.p);
     for (auto *arr : {c->d_bam, c->d_bam_rec, c->d_bam_ref, c->d_bam_len, c->d_bam_sum, c->d_bam_text, c->d_bam_comp, c->d_bam_tab, c->d_bam_seg, c->d_zout[0], c->d_zout[0] + 2, c->d_zout[0] + 4, c->d_zout[1], c->d_zout[1] + 2, c->d_zout[1] + 4}) for (int k = 0; k < 2; ++k) if (arr[k].p) cudaFree(arr[k].p);
@@ -910,26 +908,34 @@ static int host_threads()
 /* one BAM file as SAM text in device memory (slot s); defined behind BamProducer */
 static int bam_to_device_text(xm_ctx *c, const void *bam, uint64_t len, int s, uint8_t **d_text, uint64_t *text_len);
 
+/* the header and reference names of a BAM file (blocks: its bgzf_scan table): 4, 16, 64 ... leading blocks inflated on
+ * `threads` host threads until the header is complete */
+static bool bam_read_header(const uint8_t *bam, const std::vector<BgzfBlock> &blocks, uint64_t total, int threads, BamIndex &ix, std::string &err)
+{
+    for (size_t take = std::min<size_t>(blocks.size(), 4);; take = std::min(blocks.size(), take * 4)) {
+        const uint64_t bytes = take < blocks.size() ? blocks[take].out_off : total;
+        std::vector<uint8_t> buf(bytes + 16);
+        if (!bgzf_inflate(bam, blocks, 0, take, buf.data(), threads, err)) return false;
+        ix = BamIndex();
+        if (bam_index(buf.data(), bytes, ix, true, err)) return true;
+        if (take == blocks.size()) return false;
+    }
+}
+
 int xm_bam_header_text(const void *bam, uint64_t len, char *dst, uint64_t cap, uint64_t *needed)
 {
     if (!bam || !needed) return XM_ERR_ARG;
     std::string err;
     std::vector<BgzfBlock> blocks;
     uint64_t total = 0;
-    if (!bgzf_scan((const uint8_t *)bam, len, blocks, total, err)) { g_create_error = "BAM input: " + err; return XM_ERR_IO; }
-    /* inflate leading blocks until the header is complete */
-    for (size_t take = std::min<size_t>(blocks.size(), 4);; take = std::min(blocks.size(), take * 4)) {
-        const uint64_t bytes = take < blocks.size() ? blocks[take].out_off : total;
-        std::vector<uint8_t> buf(bytes + 16);
-        if (!bgzf_inflate((const uint8_t *)bam, blocks, 0, take, buf.data(), 1, err)) { g_create_error = "BAM input: " + err; return XM_ERR_IO; }
-        BamIndex ix;
-        if (bam_index(buf.data(), bytes, ix, true, err)) {
-            *needed = ix.text.size();
-            if (dst && cap >= ix.text.size()) memcpy(dst, ix.text.data(), ix.text.size());
-            return XM_OK;
-        }
-        if (take == blocks.size()) { g_create_error = "BAM input: " + err; return XM_ERR_IO; }
+    BamIndex ix;
+    if (!bgzf_scan((const uint8_t *)bam, len, blocks, total, err) || !bam_read_header((const uint8_t *)bam, blocks, total, 1, ix, err)) {
+        g_create_error = "BAM input: " + err;
+        return XM_ERR_IO;
     }
+    *needed = ix.text.size();
+    if (dst && cap >= ix.text.size()) memcpy(dst, ix.text.data(), ix.text.size());
+    return XM_OK;
 }
 
 int xm_bam_render_host(xm_ctx *c, const void *bam, uint64_t len, const void **text, uint64_t *text_len)
@@ -967,11 +973,12 @@ static bool bam_inflate_on_host()
     const char *e = getenv("XM_BAM_INFLATE");
     return e && !strcmp(e, "host");
 }
-static int upload_shard(xm_ctx *c, uint8_t *d_dst, const uint8_t *src, uint64_t n);
 
-/* BAM as a source of the chunked walk: each call inflates the next BGZF blocks on the host (thread pool), follows the
- * record chain, uploads the whole records and renders them as SAM text straight into the walk's staging buffer.  What
- * is resident at any time is one batch, not the file: the inflated size of a BAM no longer has to fit the GPU. */
+/* BAM as a source of the chunked walk.  The file is taken a window of BGZF blocks at a time (XM_BAM_WINDOW): the blocks
+ * are inflated into device memory (k_bgzf_inflate; XM_BAM_INFLATE=host: zlib on the host threads, then uploaded), the
+ * record chain is followed by k_bam_chain, and each call renders records of the window as SAM text straight into the
+ * walk's staging buffer.  What is resident at any time is one window, not the file: the inflated size of a BAM does not
+ * have to fit the GPU. */
 struct BamProducer : DevSource {
     xm_ctx *c = nullptr;
     int s = 0;
@@ -979,139 +986,12 @@ struct BamProducer : DevSource {
     uint64_t bam_len = 0;
     std::vector<BgzfBlock> blocks;
     size_t blk = 0;
-    bool have_header = false;
-    uint64_t left = 0;                  /* bytes of an incomplete record at the front of the pinned buffer */
     uint32_t n_ref = 0;
     uint8_t *d_names = nullptr;
-    /* a batch that was inflated but did not fit the room it was offered: rendered by the next call */
-    bool pending = false;
-    std::vector<uint64_t> pend_rec;
-    uint64_t pend_have = 0, pend_end = 0, full_cap = 0;
+    uint64_t full_cap = 0;              /* the walk's whole staging step: a record that does not fit it is refused */
 
-    int next_host(uint8_t *dev_dst, uint64_t max_bytes, uint64_t &n_out, bool &final, std::string &err)
-    {
-        n_out = 0; final = false;
-        if (max_bytes == 0) return XM_OK;
-        cudaStream_t st = c->be.st;
-        const uint64_t budget = std::max<uint64_t>(max_bytes / 6, 1u << 16);          /* a BAM byte renders to at most ~5 text bytes */
-        std::vector<uint64_t> rec;
-        uint64_t have = left, cursor = 0;
-        const auto t0 = std::chrono::steady_clock::now();
-        for (;;) {
-            uint64_t o = 0;
-            int rc = XM_OK;
-            bool again = false;
-            if (pending) { rec.swap(pend_rec); have = pend_have; o = pend_end; pending = false; again = true; goto render; }
-            {
-            /* the next blocks, up to the budget (at least one) */
-            size_t last = blk;
-            uint64_t add = 0;
-            while (last < blocks.size() && (last == blk || add + blocks[last].out_len <= budget)) add += blocks[last++].out_len;
-            if ((rc = reserve_host_keep(have + add + 64))) { err = c->err; return rc; }
-            if (last > blk) {
-                std::string e;
-                if (!bgzf_inflate(bam, blocks, blk, last, c->h_bam[s].p + have - blocks[blk].out_off, host_threads(), e)) { err = "BAM input: " + e; return XM_ERR_IO; }
-            }
-            have += add;
-            blk = last;
-            uint8_t *h = c->h_bam[s].p;
-            if (!have_header) {
-                BamIndex ix;
-                std::string e;
-                if (!bam_index(h, have, ix, true, e)) {
-                    if (blk < blocks.size()) continue;            /* the header goes on in the next blocks */
-                    err = "BAM input: " + e; return XM_ERR_IO;
-                }
-                have_header = true;
-                cursor = ix.first_record;
-                n_ref = (uint32_t)ix.ref_off.size() - 1;
-                const uint64_t ref_bytes = ix.ref_off.size() * 4 + ix.ref_names.size() + 16;
-                if ((rc = reserve_dev(c, c->d_bam_ref[s], ref_bytes))) { err = c->err; return rc; }
-                cudaMemcpyAsync(c->d_bam_ref[s].p, ix.ref_off.data(), ix.ref_off.size() * 4, cudaMemcpyHostToDevice, st);
-                d_names = c->d_bam_ref[s].p + ix.ref_off.size() * 4;
-                if (!ix.ref_names.empty()) cudaMemcpyAsync(d_names, ix.ref_names.data(), ix.ref_names.size(), cudaMemcpyHostToDevice, st);
-                cudaStreamSynchronize(st);
-            }
-            /* whole records in [cursor, have) */
-            o = cursor;
-            while (o + 4 <= have) {
-                const uint32_t bs = rd_u32(h + o);
-                if (bs < 32) { err = "corrupt BAM record"; return XM_ERR_IO; }
-                if (o + 4 + (uint64_t)bs > have) break;
-                rec.push_back(o);
-                o += 4 + (uint64_t)bs;
-            }
-            if (rec.empty() && blk < blocks.size()) { cursor = o; continue; }       /* a record larger than the batch: take more blocks */
-            if (blk == blocks.size() && o != have) { err = "truncated BAM record at the end of the file"; return XM_ERR_IO; }
-            }
-        render:
-            uint8_t *h = c->h_bam[s].p;
-            final = blk == blocks.size();
-            const uint64_t n = rec.size();
-            if (!again) {
-                c->bam_stats.inflate_s += std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
-                c->bam_stats.inflated_bytes += have - left;
-                c->bam_stats.records += n;
-            }
-            if (n) {
-                const uint64_t lo = rec[0], hi = o, nb = (n + 1023) / 1024;
-                for (auto &r : rec) r -= lo;
-                if ((rc = reserve_dev(c, c->d_bam[s], hi - lo + 64)) || (rc = reserve_dev(c, c->d_bam_rec[s], n * 8)) ||
-                    (rc = reserve_dev(c, c->d_bam_len[s], n * 8 + 16)) || (rc = reserve_dev(c, c->d_bam_sum[s], nb * 8 + 16))) { err = c->err; return rc; }
-                cudaEvent_t e0, e1;
-                cudaEventCreate(&e0); cudaEventCreate(&e1);
-                cudaMemcpyAsync(c->d_bam[s].p, h + lo, hi - lo, cudaMemcpyHostToDevice, st);
-                cudaMemcpyAsync(c->d_bam_rec[s].p, rec.data(), n * 8, cudaMemcpyHostToDevice, st);
-                unsigned long long *d_err = (unsigned long long *)(c->d_bam_sum[s].p + nb * 8);
-                const unsigned long long no_err = BAM_NO_ERROR;
-                cudaMemcpyAsync(d_err, &no_err, 8, cudaMemcpyHostToDevice, st);
-                BamDev B;
-                B.data = c->d_bam[s].p; B.rec = (const uint64_t *)c->d_bam_rec[s].p; B.n = n;
-                B.ref_off = (const uint32_t *)c->d_bam_ref[s].p; B.ref_names = d_names; B.n_ref = n_ref;
-                uint32_t *d_len = (uint32_t *)c->d_bam_len[s].p, *d_loff = d_len + n + (n & 1);
-                cudaEventRecord(e0, st);
-                k_bam_len<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(B, d_len, d_err);
-                k_bam_scan_blocks<<<(unsigned)nb, 1024, 0, st>>>(d_len, n, d_loff, (unsigned long long *)c->d_bam_sum[s].p);
-                std::vector<unsigned long long> sums(nb + 1);
-                cudaMemcpyAsync(sums.data(), c->d_bam_sum[s].p, (nb + 1) * 8, cudaMemcpyDeviceToHost, st);
-                if (cudaStreamSynchronize(st) != cudaSuccess) { err = "BAM length kernels failed"; return XM_ERR_CUDA; }
-                if (sums[nb] != BAM_NO_ERROR) {
-                    cudaEventDestroy(e0); cudaEventDestroy(e1);
-                    if ((sums[nb] & 0xff) == BAM_E_FLOAT) { err = "a BAM record has a float aux value (f or B:f): not rendered on the device"; return XM_ERR_UNSUPPORTED; }
-                    err = "corrupt BAM record"; return XM_ERR_IO;
-                }
-                unsigned long long run = 0;
-                for (uint64_t k = 0; k < nb; ++k) { const unsigned long long v = sums[k]; sums[k] = run; run += v; }
-                if (run > max_bytes) {
-                    cudaEventDestroy(e0); cudaEventDestroy(e1);
-                    if (max_bytes >= full_cap) { err = "BAM records render to more text than a staging step holds"; return XM_ERR_UNSUPPORTED; }
-                    /* offered less than a whole step (the walk buffer is full of carried records): keep the batch for the next call */
-                    for (auto &r : rec) r += lo;
-                    pend_rec.swap(rec); pend_have = have; pend_end = o; pending = true;
-                    final = false;
-                    return XM_OK;
-                }
-                cudaMemcpyAsync(c->d_bam_sum[s].p, sums.data(), nb * 8, cudaMemcpyHostToDevice, st);
-                k_bam_render<<<(unsigned)((n * 32 + 255) / 256), 256, 0, st>>>(B, 0, n, d_loff, (const unsigned long long *)c->d_bam_sum[s].p, dev_dst);
-                cudaEventRecord(e1, st);
-                if (cudaStreamSynchronize(st) != cudaSuccess || cudaGetLastError() != cudaSuccess) { err = "BAM render kernel failed"; return XM_ERR_CUDA; }
-                float ms = 0.f;
-                cudaEventElapsedTime(&ms, e0, e1);
-                cudaEventDestroy(e0); cudaEventDestroy(e1);
-                c->bam_stats.render_ms += ms;
-                c->bam_stats.text_bytes += run;
-                c->bam_stats.n_launches += 3;
-                n_out = run;
-            }
-            /* the incomplete record stays for the next call */
-            left = have - o;
-            if (left) memmove(h, h + o, left);
-            return XM_OK;
-        }
-    }
-
-    /* ---- the device path: windows of BGZF blocks inflated by k_bgzf_inflate, the record chain by k_bam_chain ----------- */
-    bool host_mode = false;             /* XM_BAM_INFLATE=host: zlib on host threads (the round-1 path, kept for comparison) */
+    bool host_mode = false;             /* XM_BAM_INFLATE=host: blocks inflated by zlib on the host threads */
+    std::vector<uint8_t> h_piece;       /* host mode: inflated blocks on their way to d_bam[s] */
     uint64_t inflated_total = 0;
     uint64_t skip = 0;                  /* header bytes of the inflated stream that are still ahead */
     uint64_t have_d = 0, win_end = 0;   /* inflated bytes in d_bam[s]; end of the last whole record among them */
@@ -1129,32 +1009,21 @@ struct BamProducer : DevSource {
         std::string e;
         if (!bgzf_scan(bam, bam_len, blocks, inflated_total, e)) { err = "BAM input: " + e; return XM_ERR_IO; }
         c->bam_stats.bam_bytes += bam_len;
-        if (host_mode) return XM_OK;
-        for (size_t take = std::min<size_t>(blocks.size(), 4);; take = std::min(blocks.size(), take * 4)) {
-            const uint64_t bytes = take < blocks.size() ? blocks[take].out_off : inflated_total;
-            std::vector<uint8_t> buf(bytes + 16);
-            if (!bgzf_inflate(bam, blocks, 0, take, buf.data(), host_threads(), e)) { err = "BAM input: " + e; return XM_ERR_IO; }
-            BamIndex ix;
-            if (bam_index(buf.data(), bytes, ix, true, e)) {
-                have_header = true;
-                skip = ix.first_record;
-                skip_abs = ix.first_record;
-                n_ref = (uint32_t)ix.ref_off.size() - 1;
-                const uint64_t ref_bytes = ix.ref_off.size() * 4 + ix.ref_names.size() + 16;
-                int rc;
-                if ((rc = reserve_dev(c, c->d_bam_ref[s], ref_bytes))) { err = c->err; return rc; }
-                cudaMemcpyAsync(c->d_bam_ref[s].p, ix.ref_off.data(), ix.ref_off.size() * 4, cudaMemcpyHostToDevice, c->be.st);
-                d_names = c->d_bam_ref[s].p + ix.ref_off.size() * 4;
-                if (!ix.ref_names.empty()) cudaMemcpyAsync(d_names, ix.ref_names.data(), ix.ref_names.size(), cudaMemcpyHostToDevice, c->be.st);
-                if (cudaStreamSynchronize(c->be.st) != cudaSuccess) { err = "H2D copy failed"; return XM_ERR_CUDA; }
-                return XM_OK;
-            }
-            if (take == blocks.size()) { err = "BAM input: " + e; return XM_ERR_IO; }
-        }
+        BamIndex ix;
+        if (!bam_read_header(bam, blocks, inflated_total, host_threads(), ix, e)) { err = "BAM input: " + e; return XM_ERR_IO; }
+        skip = ix.first_record;
+        skip_abs = ix.first_record;
+        n_ref = (uint32_t)ix.ref_off.size() - 1;
+        const uint64_t ref_bytes = ix.ref_off.size() * 4 + ix.ref_names.size() + 16;
+        int rc;
+        if ((rc = reserve_dev(c, c->d_bam_ref[s], ref_bytes))) { err = c->err; return rc; }
+        cudaMemcpyAsync(c->d_bam_ref[s].p, ix.ref_off.data(), ix.ref_off.size() * 4, cudaMemcpyHostToDevice, c->be.st);
+        d_names = c->d_bam_ref[s].p + ix.ref_off.size() * 4;
+        if (!ix.ref_names.empty()) cudaMemcpyAsync(d_names, ix.ref_names.data(), ix.ref_names.size(), cudaMemcpyHostToDevice, c->be.st);
+        if (cudaStreamSynchronize(c->be.st) != cudaSuccess) { err = "H2D copy failed"; return XM_ERR_CUDA; }
+        return XM_OK;
     }
 
-    /* the next window: what is left of the last one moves to the front, the next blocks are inflated behind it, the chain is
-     * followed and the text length of every record is found */
     /* blocks [lo, hi) inflated behind the `left` bytes at the front of d_bam[s] (which holds them all) */
     int inflate_blocks(size_t lo, size_t hi, uint64_t left, std::string &err)
     {
@@ -1162,6 +1031,23 @@ struct BamProducer : DevSource {
         const size_t nblk = hi - lo;
         if (!nblk) return XM_OK;
         int rc;
+        if (host_mode) {
+            /* 64 MiB of inflated bytes at a time through one host buffer: the host memory stays small whatever the window.
+             * The upload runs on the copy streams: the move of the last window's tail to the front (on st) ends first. */
+            if (cudaStreamSynchronize(st) != cudaSuccess) { err = "D2D copy failed"; return XM_ERR_CUDA; }
+            for (size_t a = lo, b; a < hi; a = b) {
+                uint64_t n = 0;
+                for (b = a; b < hi && (b == a || n + blocks[b].out_len <= (64ull << 20)); ++b) n += blocks[b].out_len;
+                if (!n) continue;                                  /* empty blocks only */
+                if (h_piece.size() < n) h_piece.resize(n);
+                std::string e;
+                if (!bgzf_inflate(bam, blocks, a, b, h_piece.data() - blocks[a].out_off, host_threads(), e)) { err = "BAM input: " + e; return XM_ERR_IO; }
+                const auto tu = std::chrono::steady_clock::now();
+                if ((rc = upload_shard(c, c->d_bam[s].p + left + (blocks[a].out_off - blocks[lo].out_off), h_piece.data(), n))) { err = c->err; return rc; }
+                c->bam_stats.upload_s += std::chrono::duration<double>(std::chrono::steady_clock::now() - tu).count();
+            }
+            return XM_OK;
+        }
         const uint64_t c0 = blocks[lo].in_off, c1 = blocks[hi - 1].in_off + blocks[hi - 1].in_len;
         if ((rc = reserve_dev(c, c->d_bam_comp[s], c1 - c0 + 64)) || (rc = reserve_dev(c, c->d_bam_tab[s], nblk * sizeof(BgzfDev) + 16))) { err = c->err; return rc; }
         const auto tu = std::chrono::steady_clock::now();
@@ -1260,14 +1146,13 @@ struct BamProducer : DevSource {
         if (cudaStreamSynchronize(st) != cudaSuccess || cudaGetLastError() != cudaSuccess) { err = "BAM length kernels failed"; return XM_ERR_CUDA; }
         c->bam_stats.render_ms += rv.ms();
         c->bam_stats.n_launches += 4;
-        if (sums[nb] != BAM_NO_ERROR) {
-            if ((sums[nb] & 0xff) == BAM_E_FLOAT) { err = "a BAM record has a float aux value (f or B:f): not rendered on the device"; return XM_ERR_UNSUPPORTED; }
-            err = "corrupt BAM record"; return XM_ERR_IO;
-        }
+        if (sums[nb] != BAM_NO_ERROR) { err = "corrupt BAM record"; return XM_ERR_IO; }
         c->bam_stats.records += n_rec;
         return XM_OK;
     }
 
+    /* the next window: what is left of the last one moves to the front, the next blocks are inflated behind it, the chain is
+     * followed and the text length of every record is found */
     int load_window(std::string &err)
     {
         cudaStream_t st = c->be.st;
@@ -1372,13 +1257,7 @@ struct BamProducer : DevSource {
         uint64_t off = 0;
         while (r_next < n_rec) {
             uint64_t n = 0;
-            bool fin = false;
-            full_cap = text_len - off;
-            const size_t keep_blk = blk;
-            blk = blocks.size();                               /* next() must not load windows */
-            rc = next(T.p + front_room + off, text_len - off, n, fin, err);
-            blk = keep_blk;
-            if (rc) return rc;
+            if ((rc = render_window(T.p + front_room + off, text_len - off, n, err))) return rc;
             if (!n) { err = "BAM shard rendering made no progress"; return XM_ERR_IO; }
             off += n;
         }
@@ -1401,19 +1280,14 @@ struct BamProducer : DevSource {
         return t - cut_off;
     }
 
-    int next(uint8_t *dev_dst, uint64_t max_bytes, uint64_t &n_out, bool &final, std::string &err) override
+    /* Up to max_bytes of text of the current window's records from r_next on into dev_dst (r_next < n_rec); n_out = 0:
+     * not even the next record fits.  Whole groups of 1024 records while they fit, then the records of the next group
+     * that still do (its offsets are read back: 4 KiB).  cut_off: text bytes of r_next's group that earlier calls
+     * rendered. */
+    int render_window(uint8_t *dev_dst, uint64_t max_bytes, uint64_t &n_out, std::string &err)
     {
-        if (host_mode) return next_host(dev_dst, max_bytes, n_out, final, err);
-        n_out = 0; final = false;
-        if (max_bytes == 0) return XM_OK;
+        n_out = 0;
         cudaStream_t st = c->be.st;
-        while (r_next == n_rec) {
-            if (blk == blocks.size()) { final = true; return XM_OK; }
-            const int rc = load_window(err);
-            if (rc) return rc;
-        }
-        /* whole groups of 1024 records while they fit, then the records of the next group that still do (its offsets
-         * are read back: 4 KiB).  cut_off: text bytes of r_next's group that earlier calls rendered. */
         const uint64_t g0 = r_next >> 10, nbw = (n_rec + 1023) / 1024;
         const uint32_t *d_len = (const uint32_t *)c->d_bam_len[s].p, *d_loff = d_len + n_rec + (n_rec & 1);
         uint64_t g = g0, bytes = 0, r_end = r_next, cut_end = cut_off;
@@ -1433,10 +1307,7 @@ struct BamProducer : DevSource {
             while (j + 1 < cnt_g && loff[j + 1] - start <= room) ++j;  /* loff[j + 1] - start: text of the records up to j */
             if (lo + j > r_end) { bytes += loff[j] - start; r_end = lo + j; cut_end = loff[j]; }
         }
-        if (r_end == r_next) {
-            if (max_bytes >= full_cap) { err = "a BAM record renders to more text than a staging step holds"; return XM_ERR_UNSUPPORTED; }
-            return XM_OK;                        /* offered less than a whole step: the walk buffer is full of carried records */
-        }
+        if (r_end == r_next) return XM_OK;
         const uint64_t cnt = r_end - r_next, ng = ((r_end - 1) >> 10) - g0 + 1;
         std::vector<unsigned long long> bases(ng);
         unsigned long long run = 0ull - cut_off;                       /* wraps: the first group's base lies before dev_dst */
@@ -1453,19 +1324,22 @@ struct BamProducer : DevSource {
         cut_off = cut_end;
         r_next = r_end;
         n_out = bytes;
-        final = r_next == n_rec && blk == blocks.size();
         return XM_OK;
     }
-    /* pinned buffer of the inflated batch, grown without losing the bytes at its front */
-    int reserve_host_keep(uint64_t need)
+
+    /* the walk's source: windows are loaded while the current one is spent */
+    int next(uint8_t *dev_dst, uint64_t max_bytes, uint64_t &n_out, bool &final, std::string &err) override
     {
-        HostBuf &b = c->h_bam[s];
-        if (need <= b.cap && b.p) return XM_OK;
-        uint8_t *np_ = nullptr;
-        const uint64_t cap = std::max<uint64_t>(need, b.cap * 2);
-        if (cudaHostAlloc((void **)&np_, cap + 64, cudaHostAllocDefault) != cudaSuccess) { cudaGetLastError(); return fail(c, XM_ERR_NOMEM, "cudaHostAlloc: out of memory"); }
-        if (b.p) { if (left) memcpy(np_, b.p, left); cudaFreeHost(b.p); }
-        b.p = np_; b.cap = cap;
+        n_out = 0; final = false;
+        if (max_bytes == 0) return XM_OK;
+        int rc;
+        while (r_next == n_rec) {
+            if (blk == blocks.size()) { final = true; return XM_OK; }
+            if ((rc = load_window(err))) return rc;
+        }
+        if ((rc = render_window(dev_dst, max_bytes, n_out, err))) return rc;
+        if (!n_out && max_bytes >= full_cap) { err = "a BAM record renders to more text than a staging step holds"; return XM_ERR_UNSUPPORTED; }
+        final = r_next == n_rec && blk == blocks.size();      /* n_out = 0 and not final: the walk buffer is full of carried records */
         return XM_OK;
     }
 };
@@ -1481,38 +1355,23 @@ static int bam_to_device_text(xm_ctx *c, const void *bam, uint64_t len, int s, u
     if (rc) return fail(c, rc, err);
     DevBuf &T = c->d_bam_text[s];
     uint64_t off = 0;
-    if (p.host_mode) {
-        /* the host path renders what it is offered room for: offer the most a BAM byte can become */
-        if ((rc = reserve_dev(c, T, p.inflated_total * 6 + 4096))) return rc;
-        p.full_cap = T.cap;
-        for (;;) {
-            uint64_t n = 0;
-            bool final = false;
-            if ((rc = p.next(T.p + off, T.cap - off, n, final, err))) return fail(c, rc, err);
-            off += n;
-            if (final) break;
+    for (;;) {
+        while (p.r_next == p.n_rec && p.blk < p.blocks.size()) if ((rc = p.load_window(err))) return fail(c, rc, err);
+        const uint64_t want = p.window_text_left();
+        if (!want) break;
+        if (off + want > T.cap || !T.p) {                   /* grow, keeping what is rendered */
+            uint8_t *np_ = nullptr;
+            const uint64_t cap = std::max<uint64_t>(off + want, T.cap * 2);
+            if (cudaMalloc((void **)&np_, cap + 64) != cudaSuccess) { cudaGetLastError(); return fail(c, XM_ERR_NOMEM, "cudaMalloc: out of memory"); }
+            if (off) { cudaMemcpyAsync(np_, T.p, off, cudaMemcpyDeviceToDevice, c->be.st); cudaStreamSynchronize(c->be.st); }
+            if (T.p) cudaFree(T.p);
+            T.p = np_; T.cap = cap;
         }
-    } else {
-        for (;;) {
-            while (p.r_next == p.n_rec && p.blk < p.blocks.size()) if ((rc = p.load_window(err))) return fail(c, rc, err);
-            const uint64_t want = p.window_text_left();
-            if (!want) break;
-            if (off + want > T.cap || !T.p) {                   /* grow, keeping what is rendered */
-                uint8_t *np_ = nullptr;
-                const uint64_t cap = std::max<uint64_t>(off + want, T.cap * 2);
-                if (cudaMalloc((void **)&np_, cap + 64) != cudaSuccess) { cudaGetLastError(); return fail(c, XM_ERR_NOMEM, "cudaMalloc: out of memory"); }
-                if (off) { cudaMemcpyAsync(np_, T.p, off, cudaMemcpyDeviceToDevice, c->be.st); cudaStreamSynchronize(c->be.st); }
-                if (T.p) cudaFree(T.p);
-                T.p = np_; T.cap = cap;
-            }
-            p.full_cap = want;
-            uint64_t n = 0;
-            bool final = false;
-            if ((rc = p.next(T.p + off, want, n, final, err))) return fail(c, rc, err);
-            off += n;
-        }
-        if (!T.p && (rc = reserve_dev(c, T, 64))) return rc;
+        uint64_t n = 0;                                     /* offered the whole rest of the window: renders all of it */
+        if ((rc = p.render_window(T.p + off, want, n, err))) return fail(c, rc, err);
+        off += n;
     }
+    if (!T.p && (rc = reserve_dev(c, T, 64))) return rc;
     *d_text = T.p;
     *text_len = off;
     return XM_OK;

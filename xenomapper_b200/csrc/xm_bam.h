@@ -165,7 +165,7 @@ struct BamDev {
     uint32_t n_ref;
 };
 constexpr unsigned long long BAM_NO_ERROR = ~0ull;
-enum { BAM_E_FLOAT = 1, BAM_E_CORRUPT = 2 };
+enum { BAM_E_CORRUPT = 2 };
 
 #if defined(__CUDACC__)
 __device__ __forceinline__ uint32_t ld_u16(const uint8_t *p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8); }

@@ -188,7 +188,7 @@ struct FdFeeder {
     }
 };
 
-/* a source that puts whole lines straight into a device buffer (BAM input: inflate on the host, render on the GPU) */
+/* a source that puts whole lines straight into a device buffer (BAM input: records rendered as SAM text on the GPU) */
 struct DevSource {
     virtual ~DevSource() {}
     /* up to max_bytes of SAM text into dev_dst; n = bytes written, final = the stream ends with them.  Returns an xm_status. */
