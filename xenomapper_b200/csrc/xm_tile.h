@@ -18,8 +18,13 @@
  *
  * A line belongs to the tile that holds its first byte.  The window staged in
  * shared memory extends HALO bytes to both sides so that the last owned line
- * and the line before the first owned one are normally inside it; lines that
- * are not are handled through global memory by the exact byte-wise path.
+ * and the line before the first owned one are normally inside it.  Lines that
+ * are not take the exact byte-wise path through global memory: the last owned
+ * line when it ends past the window, and the halo line when it starts before
+ * it -- its start is found by walking back from the window, it is parsed from
+ * global memory, its QNAME is compared with the first owned line's through
+ * global memory (prev_name_equal) and a pair unit that begins with it is copied
+ * from there.  A tile that one line covers owns no line.
  *
  * Byte classes.  Two exact masks are built per tile: W (byte < 0x21 or
  * >= 0x80: every separator, control and non-ASCII byte) and T (tab).  Line
@@ -320,11 +325,20 @@ inline void emu_lookback2(unsigned long long *chain, uint32_t tile, unsigned lon
 }
 #endif
 
+/* names_equal for a previous QNAME that may start before the window (the halo line of a tile whose first owned line
+ * is preceded by a line longer than the halo): names_equal's word-wise path takes both names to start inside it */
+XM_HD bool prev_name_equal(const Reader &rd, uint64_t prev_qs, uint32_t prev_qlen, uint64_t qs, uint32_t qlen)
+{
+    if (prev_qs >= rd.g0) return names_equal(rd, prev_qs, prev_qlen, qs, qlen);
+    const Reader rg{rd.win, rd.glob, 0, 0u, rd.len};      /* every byte from global memory */
+    return names_equal(rg, prev_qs, prev_qlen, qs, qlen);
+}
+
 /* is line i (QNAME in th.L) the first of its run of equal QNAMEs?  prev = (qs, qlen, h1, h2) of the line before */
 XM_HD bool run_head(const Reader &rd, const LineRec &L, const uint4 prev, uint64_t prev_qs_global)
 {
     if (prev.y != L.qlen || prev.z != L.h1 || prev.w != L.h2) return true;
-    return !names_equal(rd, prev_qs_global, prev.y, rd.g0 + L.qs, L.qlen);
+    return !prev_name_equal(rd, prev_qs_global, prev.y, rd.g0 + L.qs, L.qlen);
 }
 
 /* ---- front end shared by both kernels: stage, mask, index, parse --------- */
@@ -497,7 +511,7 @@ XM_HD void front_end(TileCtx<C> &T, ThreadState<C> &th_, const StreamBuf &B, int
         th.yoff = 0;                    /* 1 = the aux half of the line is done by the partner thread */
         th.sin = 0xffffffffu;
         const bool mine = (uint32_t)tid < fr.nlines;
-        bool halo = false, farline = false, clean = false, tjob = false;
+        bool halo = false, farline = false, clean = false, tjob = false, split_line = false;
         int s = 0, e = 0;
         uint64_t gs = 0;
         FastCtx fc;
@@ -509,9 +523,11 @@ XM_HD void front_end(TileCtx<C> &T, ThreadState<C> &th_, const StreamBuf &B, int
                 const int s0 = (int)T.m.lstart[0];
                 gs = prev_line_start(T.m.nlm, B.p, geo.g0, s0);
                 if (!dirty && gs > geo.g0 && T.m.win[gs - geo.g0 - 1] != '\n') {
-                    /* the candidate before the halo line is not a newline: find its real start byte-wise */
+                    /* the candidate before the halo line is not a newline: find its real start byte-wise.  The line
+                     * holds that candidate (a space, a CR ...), so the mask-driven parse does not apply to it. */
                     --gs;
                     while (gs > 0 && rd_.at(gs - 1) != '\n') --gs;
+                    split_line = true;
                 }
                 farline = gs < geo.g0;
                 if (farline) { rd_.wbytes = 0; rd_.g0 = gs; }       /* read it all from global memory */
@@ -527,7 +543,7 @@ XM_HD void front_end(TileCtx<C> &T, ThreadState<C> &th_, const StreamBuf &B, int
             gs = geo.g0 + (uint64_t)s;
         }
         if (mine || halo) {
-            if (!dirty && !farline) clean = fast_head(M_, s, e, th.L, fc);
+            if (!dirty && !farline && !split_line) clean = fast_head(M_, s, e, th.L, fc);
             if (!clean) {               /* out of line: keep its operands off this thread's registers' stack */
                 const Reader rg_ = rd_;
                 LineRec G;
@@ -902,7 +918,7 @@ XM_HD void classify_tile(TileCtx<C> &T, const ClassifyArgs &a, uint32_t tile)
                 if (fire) {
                     const Reader rd_{T.m.win, a.P.p, fr.geo.g0, fr.geo.wbytes, a.P.len};
                     const uint64_t pq = (i == 0) ? T.m.scr64[S64_HALO_QS] : fr.geo.g0 + pv.x;
-                    fire = names_equal(rd_, pq, pv.y, fr.geo.g0 + L.qs, L.qlen);
+                    fire = prev_name_equal(rd_, pq, pv.y, fr.geo.g0 + L.qs, L.qlen);
                 }
                 if (fire && !own_ec) {                      /* the assert fires before the unit is looked at */
                     const int pst = (int)((pv.w >> 24) & 7u), pev = (int)((pv.w >> 27) & 7u), pevs = (int)(pv.w >> 31);
